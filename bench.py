@@ -3,7 +3,7 @@
 headline workload: synthetic 1,048,576-point foam, one 1920x1080 frame, Q = 2 depth
 quantiles, sh_degree 3, fp32 (config 4; SURVEY.md §8d).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over the frame: scene re-layout (points/attributes
@@ -13,6 +13,9 @@ trace_backward (+ one all-reduce of the per-point gradient accumulator when N > 
 the step's inputs in pinned HOST memory (H2D inside the timed region) and the loss read back.
 Rank 0 prints ONE JSON line.  The oracle is used only by the cpu_baseline leg and by
 --impl reference (which times the reference's OWN CUDA kernels from oracle/_ref).
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs) so that two builds can be compared.
+The run writes nothing into the source tree (which may be read-only): the foam cache lives under the system's
+temporary directory.
 """
 from __future__ import annotations
 
@@ -22,9 +25,12 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 
-import numpy as np
+sys.dont_write_bytecode = True
+
+import numpy as np  # noqa: E402
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -38,12 +44,12 @@ FOV = 0.9
 # ----------------------------------------------------------------------------- workload
 def load_or_build_foam(num_points: int, log):
     """Delaunay adjacency costs ~35 s/Mpoint on one core (and on an N-GPU box every GPU is charged while rank 0
-    builds it).  Two caches: the full foam under .bench_cache/ (box-local), and the packed ADJACENCY only under
-    foam_cache/ (17 MB per Mpoint; git-ignored but shipped to the GPU box) -- points and attributes are regenerated
+    builds it).  Two caches: the full foam under the temporary directory (machine-local), and the packed ADJACENCY
+    only under foam_cache/ (17 MB per Mpoint; git-ignored, read if present) -- points and attributes are regenerated
     from the seed in seconds."""
     from radfoam_b200 import foam
 
-    cache_dir = os.path.join(ROOT, ".bench_cache")
+    cache_dir = os.path.join(tempfile.gettempdir(), f"radfoam_b200_bench_cache_{os.getuid()}")
     path = os.path.join(cache_dir, f"foam_{num_points}.npz")
     if os.path.exists(path):
         z = np.load(path)
@@ -103,6 +109,45 @@ def make_frame(f, width: int, height: int):
     grad_depth = (rng.normal(size=(height, width, 2)) * 1e-4).astype(np.float32)
     target = rng.uniform(0.0, 1.0, size=(height, width, 4)).astype(np.float32)
     return dict(rays=rays, start=start, dq=dq, grad_rgba=grad_rgba, grad_depth=grad_depth, target=target)
+
+
+DUMP_RAYS, DUMP_POINTS = 131_072, 131_072  # sampled rows: ~36 MB for the headline workload
+
+
+def sample_outputs(outputs: dict, ray_shape: tuple, num_points: int) -> dict:
+    """What one step returned, as float32 / float64 host arrays of at most DUMP_RAYS rays and DUMP_POINTS points.  The
+    rows are a fixed, seeded sample (the same for every run with the same arguments); their indices are included as
+    ray_index and point_index.  ray_index indexes the flattened per-ray batch the step traced: the whole image on one
+    GPU; with --gpus N > 1, rank 0 writes the dump and its batch is rank 0's shard (its interleaved 8-row bands), while
+    the gradients, reduced over all ranks, are the whole step's.  Integer outputs are stored as float64, which holds
+    uint32 exactly.  ray_grad is left out: the path allocates it but never writes it."""
+    import torch
+
+    out = {}
+    for name, t in sorted(outputs.items()):
+        if name == "ray_grad" or t is None:
+            continue
+        per_ray = tuple(t.shape[:len(ray_shape)]) == tuple(ray_shape)
+        assert per_ray or t.shape[0] == num_points, (name, tuple(t.shape))
+        rows = t.reshape(-1, *t.shape[len(ray_shape):]) if per_ray else t
+        key, limit = ("ray_index", DUMP_RAYS) if per_ray else ("point_index", DUMP_POINTS)
+        if key not in out:
+            count = rows.shape[0]
+            idx = np.arange(count) if count <= limit else np.sort(
+                np.random.default_rng(1).choice(count, size=limit, replace=False))
+            out[key] = idx.astype(np.float64)
+        rows = rows.detach().index_select(0, torch.from_numpy(out[key].astype(np.int64)).to(rows.device))
+        if rows.is_floating_point():
+            out[name] = rows.float().cpu().numpy()
+        else:
+            out[name] = rows.to(torch.int64).cpu().numpy().astype(np.float64)
+    return out
+
+
+def dump_outputs(directory: str, arrays: dict):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -440,13 +485,16 @@ def run_ours(args):
     fwd_ms, bwd_ms = [], []
     ev0.record()
     for _ in range(args.steps):
-        step_device()
+        last_step = step_device()
         if args.kernel_times:
             fwd_ms.append(pipe.last_kernel_ms("forward"))
             bwd_ms.append(pipe.last_kernel_ms("backward"))
     ev1.record()
     barrier(world)
     total_ms = max_over_ranks(ev0.elapsed_time(ev1), world)
+    dumped = (sample_outputs(dict(last_step[0], **last_step[1]), dv["rays"].shape[:-1], points.shape[0])
+              if args.dump_outputs else None)
+    del last_step
     clocks = sampler.stop() if sampler else None
     launches = rp.launch_count()
     # per-phase durations from a separate short pass (events between the phases would serialise the timed loop)
@@ -632,6 +680,8 @@ def run_ours(args):
         line["e2e"]["diag"] = {"step_wall_ms": graph_e2e["wall_stats"], "eager": e2e_diag}
     elif graph_e2e:
         line["e2e"]["cuda_graph_unavailable"] = graph_e2e.get("error")
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     print(json.dumps(line), flush=True)
 
 
@@ -850,10 +900,13 @@ def run_reference(args):
     torch.cuda.synchronize()
     ev0.record()
     for _ in range(args.steps):
-        step_device()
+        last_step = step_device()
     ev1.record()
     torch.cuda.synchronize()
     ms_per_step = ev0.elapsed_time(ev1) / args.steps
+    dumped = (sample_outputs(dict(last_step[0], **last_step[1]), dv["rays"].shape[:-1], points.shape[0])
+              if args.dump_outputs else None)
+    del last_step
     clocks = sampler.stop()
     run_e2e(2)
     torch.cuda.synchronize()
@@ -883,6 +936,8 @@ def run_reference(args):
                 "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": 4, "loss": loss_val,
                 "h2d_ms_per_step": h2d_ms, "h2d_overlapped": True},
     }
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     print(json.dumps(line), flush=True)
 
 
@@ -900,7 +955,12 @@ def main():
                     help="single GPU only: trace rank 0's shard of an N-way ray split (profiling aid)")
     ap.add_argument("--kernel-times", action="store_true",
                     help="read per-kernel event timings inside the timed loop (serialises it)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs (a fixed sample of rays and points) as DIR/<name>.npy; "
+                         "with --gpus N > 1, rank 0's rays only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

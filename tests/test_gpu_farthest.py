@@ -1,10 +1,11 @@
 """GPU parity of farthest_neighbor (SURVEY.md §8f.4) through the public wrapper -> ctypes -> C ABI, against the
-CPU oracle and, when oracle/_ref was built, the reference's own kernel.  Bar: both outputs bit-exact (integers,
+CPU oracle and the reference's own kernel (its outputs stored in tests/golden/reference/kernels.npz).  Bar: both outputs bit-exact (integers,
 and floats -- IEEE sqrt/divide with the fma association pinned; NaNs match as NaNs)."""
 import numpy as np
 import pytest
 
 import common
+import refdata
 
 pytestmark = pytest.mark.gpu
 
@@ -48,17 +49,11 @@ def test_matches_oracle_bit_exact(torch_cuda, make):
 
 @pytest.mark.parametrize("make", ["edge", "scene200k"])
 def test_matches_reference_kernel_bit_exact(torch_cuda, make):
-    from oracle import ref_gpu
-
-    if not ref_gpu.available():
-        pytest.skip("oracle/_ref not built")
-    torch = torch_cuda
     f = common.farthest_edge_case() if make == "edge" else common.scene_case(200000, 8, 8, 0).foam
-    idx, radius = ours(torch, f)
-    r_idx, r_radius = ref_gpu.farthest_neighbor(dev(torch, f.points), dev(torch, f.adjacency), dev(torch, f.offsets))
-    torch.cuda.synchronize()
-    assert np.array_equal(idx, r_idx.cpu().numpy())
-    common.assert_same_floats(radius, r_radius.cpu().numpy())
+    idx, radius = ours(torch_cuda, f)
+    ref = refdata.reference(f"farthest_{make}", (f.points, f.adjacency, f.offsets))
+    refdata.assert_equal(idx, ref["indices"], "indices")
+    refdata.assert_equal(radius, ref["radius"], "radius")  # bit for bit, any NaN matching any NaN
 
 
 def test_validation_and_empty(torch_cuda):

@@ -1,10 +1,11 @@
 """BASELINE.json-sized cases on the GPU (config 2: ~0.5 M points, one 1920x1080 frame), checked
-through size-independent properties of the path plus, when oracle/_ref is present, against the
-reference's own kernels.  The foam build (Qhull) dominates the run time (~20 s)."""
+through size-independent properties of the path plus against the reference's own kernels (their outputs stored in
+tests/golden/reference/kernels.npz).  The foam build (Qhull) dominates the run time (~20 s)."""
 import numpy as np
 import pytest
 
 import common
+import refdata
 
 pytestmark = pytest.mark.gpu
 
@@ -12,13 +13,8 @@ N_POINTS = 524_288
 W, H = 1920, 1080
 
 
-@pytest.fixture(scope="module")
-def world():
-    import torch
-
-    if not torch.cuda.is_available():
-        pytest.skip("no CUDA device")
-    import radfoam_b200
+def inputs(torch):
+    """The seeded frame: scene tensors, rays, start cells, quantiles and upstream gradients on the GPU."""
     from radfoam_b200 import foam
 
     f = foam.scene_foam(N_POINTS)
@@ -30,8 +26,23 @@ def world():
     g = rng.normal(size=(H, W, 4)).astype(np.float32)
     gd = (rng.normal(size=(H, W, 2)) * 1e-4).astype(np.float32)
     d = lambda a: torch.from_numpy(np.ascontiguousarray(a)).cuda()  # noqa: E731
-    w = dict(torch=torch, foam=f, scene=[d(f.points), d(f.attributes), d(f.adjacency), d(f.offsets)],
-             rays=d(rays), start=d(start), dq=d(dq), g=d(g), gd=d(gd), pipe=radfoam_b200.create_pipeline(3))
+    return dict(foam=f, scene=[d(f.points), d(f.attributes), d(f.adjacency), d(f.offsets)],
+                rays=d(rays), start=d(start), dq=d(dq), g=d(g), gd=d(gd))
+
+
+def inputs_of(w):
+    return w["scene"], w["rays"], w["start"], w["dq"], w["g"], w["gd"]
+
+
+@pytest.fixture(scope="module")
+def world():
+    import torch
+
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    import radfoam_b200
+
+    w = dict(inputs(torch), torch=torch, pipe=radfoam_b200.create_pipeline(3))
     w["pipe"].record_tape = False
     w["fwd"] = w["pipe"].trace_forward(*w["scene"], w["rays"], w["start"], depth_quantiles=w["dq"])
     return w
@@ -97,19 +108,12 @@ def test_backward_linear_additive_and_tape_equal(world):
 
 
 def test_matches_reference_kernels_at_full_size(world):
-    from oracle import ref_gpu
-
-    if not ref_gpu.available():
-        pytest.skip("oracle/_ref not built")
-    torch = world["torch"]
-    rf = ref_gpu.trace_forward(*world["scene"], world["rays"], world["start"], world["dq"])
-    fwd = world["fwd"]
-    assert torch.equal(rf["num_intersections"], fwd["num_intersections"])   # bit-exact traversal
-    assert torch.equal(rf["depth_indices"], fwd["depth_indices"])
-    assert float((rf["rgba"] - fwd["rgba"]).abs().max()) <= 1e-5
-    assert float((rf["depth"] - fwd["depth"]).abs().max()) <= 1e-5 * float(fwd["depth"].abs().max())
-    rb = ref_gpu.trace_backward(*world["scene"], world["rays"], world["start"], rf["rgba"], world["g"],
-                                world["dq"], rf["depth_indices"], world["gd"])
+    ref = refdata.reference("config2_512k_1080p", inputs_of(world))
+    fwd = {k: v.cpu().numpy() for k, v in world["fwd"].items()}
+    refdata.assert_equal(fwd["num_intersections"], ref["num_intersections"], "num_intersections")  # bit-exact
+    refdata.assert_equal(fwd["depth_indices"], ref["depth_indices"], "depth_indices")
+    refdata.assert_close(fwd["rgba"], ref["rgba"], "rgba", rtol=0, atol=1e-5)
+    refdata.assert_close(fwd["depth"], ref["depth"], "depth", rtol=0, atol=1e-5 * float(np.abs(fwd["depth"]).max()))
     ours = _bwd(world)
     for k in ("points_grad", "attr_grad"):
-        assert common.grad_error(ours[k].cpu().numpy(), rb[k].cpu().numpy()) < 1e-5
+        assert refdata.grad_error(ours[k].cpu().numpy(), ref[k]) < 1e-5

@@ -1,10 +1,12 @@
 """Tie-heavy differential cases (tests/fuzz_cases.py) on the device: the sm_100a path through Pipeline -> ctypes ->
-C ABI against the reference's own kernels (oracle/_ref) on the same GPU.  Forward outputs must be identical value for
+C ABI against the reference's own kernels, through their outputs stored in tests/golden/reference/kernels.npz (whole
+forward outputs by hash; gradients at their largest and a spread of other entries: tests/refdata.py).  Forward outputs must be identical value for
 value (integers and floats: the arithmetic of the walk is pinned to the reference's instruction sequence, and ties are
 where a different association would pick another face); gradients within 2e-5 of max|ref| (float scatter-adds in both)
 with identical non-finite patterns.  Odd seeds replay the recorded walk tape, even seeds re-walk.
 
-`python tests/test_gpu_fuzz.py FIRST_SEED COUNT` runs a longer campaign on a GPU box."""
+`python tests/test_gpu_fuzz.py FIRST_SEED COUNT` runs a longer campaign: seeds without stored outputs are compared
+with the reference's kernels run live, which needs oracle/_ref (built where the original project's sources are)."""
 import os
 import sys
 
@@ -15,32 +17,50 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import common  # noqa: E402
 import fuzz_cases  # noqa: E402
+import refdata  # noqa: E402
 import test_gpu_parity as parity  # noqa: E402
 from test_gpu_parity import torch_cuda  # noqa: E402,F401  (fixture)
 
 pytestmark = pytest.mark.gpu
 
 
+def live_reference(case, kw):
+    """The reference's kernels run now, on every entry (oracle/_ref must have been built)."""
+    from oracle import ref_gpu
+
+    if not ref_gpu.available():
+        raise SystemExit("no stored reference outputs for this seed (0-239 are stored), and oracle/_ref was not built "
+                         "to run the reference's kernels live")
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+    import make_golden_reference
+
+    full = dict(weight_threshold=0.001, max_intersections=1024)
+    full.update(kw)
+    return {k: refdata.Output.of(v) for k, v in make_golden_reference.run_ref(case, **full).items()}
+
+
 def check_seeds(torch, seeds):
     """-> (failures [(seed, scene kind, ray kind, [what differs])], {(scene kind, ray kind)} covered)."""
     failures, seen = [], set()
+    stored = refdata.stored_cases()
     for seed in seeds:
         scene_kind, ray_kind, f, rays, start, dq, kw = fuzz_cases.make_case(seed)
         seen.add((scene_kind, ray_kind))
         case = common.Case(f, rays, start, dq, seed=seed)
-        full = dict(weight_threshold=0.001, max_intersections=1024)
-        full.update(kw)
         got = parity.run_ours(torch, case, tape=bool(seed & 1), **kw)
-        ref = parity.run_ref_gpu(torch, case, **full)
+        if f"fuzz{seed}" in stored:
+            ref = refdata.reference(f"fuzz{seed}", refdata.case_inputs(case) + (kw,))
+        else:
+            ref = live_reference(case, kw)
         what = []
         for k in ("num_intersections", "depth_indices", "rgba", "depth"):
-            if k in ref and not np.array_equal(got[k], ref[k], equal_nan=got[k].dtype.kind == "f"):
+            if k in ref and not ref[k].equal(got[k]):
                 what.append(k)
         for k in ("points_grad", "attr_grad"):
-            if common.nonfinite_mismatch(got[k], ref[k]):
+            if not ref[k].same_nonfinite(got[k]):
                 what.append(k + " non-finite pattern")
-            elif common.grad_error(got[k], ref[k]) > 2e-5:
-                what.append("%s %.2e" % (k, common.grad_error(got[k], ref[k])))
+            elif refdata.grad_error(got[k], ref[k]) > 2e-5:
+                what.append("%s %.2e" % (k, refdata.grad_error(got[k], ref[k])))
         if what:
             failures.append((seed, scene_kind, ray_kind, what))
     return failures, seen
@@ -65,11 +85,11 @@ def test_rays_traced_alone_with_threshold_zero(torch_cuda):  # noqa: F811
     for i in range(0, rays.shape[0], 2):
         case = common.Case(f, rays[i:i + 1], start[i:i + 1], dq[i:i + 1], seed=3736)
         case.grad_rgba, case.grad_depth = whole.grad_rgba[i:i + 1], whole.grad_depth[i:i + 1]
-        ref = parity.run_ref_gpu(torch_cuda, case, weight_threshold=0.0, max_intersections=1024)
+        ref = refdata.reference(f"fuzz3736_ray{i}", refdata.case_inputs(case) + (kw,))
         got = parity.run_ours(torch_cuda, case, tape=bool(i & 2), **kw)
-        assert np.array_equal(got["rgba"], ref["rgba"]) and np.array_equal(got["depth"], ref["depth"])
-        worst = max(worst, common.grad_error(got["points_grad"], ref["points_grad"]),
-                    common.grad_error(got["attr_grad"], ref["attr_grad"]))
+        assert ref["rgba"].equal(got["rgba"]) and ref["depth"].equal(got["depth"])
+        worst = max(worst, refdata.grad_error(got["points_grad"], ref["points_grad"]),
+                    refdata.grad_error(got["attr_grad"], ref["attr_grad"]))
     assert worst <= 1e-5, worst
 
 

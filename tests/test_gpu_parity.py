@@ -1,17 +1,20 @@
 """GPU parity tests proper: the hand-written sm_100a path, called through the public
 Pipeline API -> ctypes -> C ABI, against
   (a) the CPU oracle (oracle/radfoam_oracle.c), and
-  (b) the reference's own kernels (oracle/_ref), when that library was built.
+  (b) the reference's own kernels, through their outputs stored in tests/golden/reference/kernels.npz
+      (tests/refdata.py; made by tests/golden/make_golden_reference.py).
 Bars (BASELINE.json north_star): integer outputs bit-exact; floats within 1e-5; gradients
 within 1e-5 of max|ref| (they are float scatter-adds, order-nondeterministic in the reference)."""
+import os
+
 import numpy as np
 import pytest
 
 import common
+import refdata
 
 pytestmark = pytest.mark.gpu
 
-FLOAT_TOL = dict(rtol=1e-5, atol=1e-5)
 GRAD_TOL = 1e-5
 
 
@@ -81,40 +84,6 @@ def run_cpu_oracle(case, attr_dtype="float32", weight_threshold=0.001, max_inter
                                          fwd["rgba"], g, case.quantiles, fwd.get("depth_indices"),
                                          case.grad_depth, ray_error, weight_threshold, max_intersections))
     return out
-
-
-def run_ref_gpu(torch, case, attr_dtype="float32", weight_threshold=0.001, max_intersections=1024,
-                return_contribution=False, backward=True, ray_error=None):
-    from oracle import ref_gpu
-
-    if not ref_gpu.available():
-        pytest.skip("oracle/_ref/libradfoam_ref.so not built")
-    f = case.foam
-    half = attr_dtype == "float16"
-    attrs = f.attributes.astype(np.float16) if half else f.attributes
-    scene = [to_dev(torch, x) for x in (f.points, attrs, f.adjacency, f.offsets)]
-    rays_d, start_d, dq_d = to_dev(torch, case.rays), to_dev(torch, case.start), to_dev(torch, case.quantiles)
-    fwd = ref_gpu.trace_forward(*scene, rays_d, start_d, dq_d, weight_threshold, max_intersections,
-                                return_contribution)
-    out = {k: v.cpu().numpy() for k, v in fwd.items()}
-    if backward:
-        g = case.grad_rgba.astype(np.float16) if half else case.grad_rgba
-        bwd = ref_gpu.trace_backward(*scene, rays_d, start_d, fwd["rgba"], to_dev(torch, g), dq_d,
-                                     fwd.get("depth_indices"), to_dev(torch, case.grad_depth),
-                                     to_dev(torch, ray_error), weight_threshold, max_intersections)
-        out.update({k: v.cpu().numpy() for k, v in bwd.items() if k != "ray_grad"})
-    torch.cuda.synchronize()
-    return out
-
-
-def assert_forward_equal(got, ref, exact_floats=False):
-    assert np.array_equal(got["num_intersections"], ref["num_intersections"]), "num_intersections"
-    if "depth_indices" in ref:
-        assert np.array_equal(got["depth_indices"], ref["depth_indices"]), "depth_indices"
-        np.testing.assert_allclose(got["depth"], ref["depth"], **FLOAT_TOL)
-    np.testing.assert_allclose(got["rgba"].astype(np.float32), ref["rgba"].astype(np.float32), **FLOAT_TOL)
-    if exact_floats:
-        assert np.array_equal(got["rgba"], ref["rgba"]), "rgba not bit-identical"
 
 
 def assert_matches_cpu_oracle(got, ref, case, grads=True):
@@ -190,6 +159,13 @@ def test_prefetch_adjacent_diff_bit_exact(torch_cuda):
 
 
 # ------------------------------------------------------------------ vs the reference's own kernels
+LARGE_CASES = {
+    "scene60k_outside": lambda: common.scene_case(num_points=60000, width=320, height=200),
+    "scene60k_inside": lambda: common.scene_case(num_points=60000, width=320, height=200, inside=True),
+    "random60k_100k": lambda: common.random_ray_case(num_points=60000, num_rays=100000),
+}
+
+
 @pytest.fixture(params=["cached", "direct"])
 def bwd_mode(request, monkeypatch):
     """Both backward kernels (warp-aggregated shared-memory cache / direct reductions)."""
@@ -201,50 +177,57 @@ def bwd_mode(request, monkeypatch):
 def test_config1_matches_reference_kernels(torch_cuda, deg, bwd_mode):
     case = common.config1(deg, 2)
     got = run_ours(torch_cuda, case, return_contribution=True)
-    ref = run_ref_gpu(torch_cuda, case, return_contribution=True)
-    assert_forward_equal(got, ref)
-    np.testing.assert_allclose(got["contribution"], ref["contribution"], rtol=1e-5, atol=1e-6)
-    assert_grads_close(got, ref)
+    ref = refdata.reference(f"config1_deg{deg}_q2", refdata.case_inputs(case))
+    refdata.assert_forward_equal(got, ref)
+    refdata.assert_close(got["contribution"], ref["contribution"], "contribution", rtol=1e-5, atol=1e-6)
+    refdata.assert_grads_close(got, ref, GRAD_TOL)
 
 
 @pytest.mark.parametrize("inside", [False, True])
 def test_scene_matches_reference_kernels(torch_cuda, inside, bwd_mode):
-    case = common.scene_case(num_points=60000, width=320, height=200, inside=inside)
+    name = "scene60k_inside" if inside else "scene60k_outside"
+    case = LARGE_CASES[name]()
+    ref = refdata.reference(name, refdata.case_inputs(case))
     got = run_ours(torch_cuda, case)
-    ref = run_ref_gpu(torch_cuda, case)
-    assert_forward_equal(got, ref)
-    # the reference's own run-to-run scatter-add noise, for context
-    ref2 = run_ref_gpu(torch_cuda, case)
-    noise = max(common.grad_error(ref2[k], ref[k]) for k in ("points_grad", "attr_grad"))
-    ours = max(common.grad_error(got[k], ref[k]) for k in ("points_grad", "attr_grad"))
+    refdata.assert_forward_equal(got, ref)
+    # the reference's own run-to-run scatter-add noise (measured when the reference outputs were stored)
+    noise = ref["noise"]
+    ours = max(refdata.grad_error(got[k], ref[k]) for k in ("points_grad", "attr_grad"))
     print(f"grad error vs reference {ours:.2e}; reference self-noise {noise:.2e}")
     assert ours <= max(GRAD_TOL, 4 * noise)
 
 
 def test_random_ray_batch_matches_reference_kernels(torch_cuda, bwd_mode):
-    case = common.random_ray_case(num_points=60000, num_rays=100000)
-    got, ref = run_ours(torch_cuda, case), run_ref_gpu(torch_cuda, case)
-    assert_forward_equal(got, ref)
-    assert_grads_close(got, ref)
+    case = LARGE_CASES["random60k_100k"]()
+    got, ref = run_ours(torch_cuda, case), refdata.reference("random60k_100k", refdata.case_inputs(case))
+    refdata.assert_forward_equal(got, ref)
+    refdata.assert_grads_close(got, ref, GRAD_TOL)
 
 
 def test_cpu_oracle_matches_reference_kernels(torch_cuda):
     """Pins the restatement (and the Eigen shim) against the reference source itself."""
-    case = common.scene_case(num_points=60000, width=320, height=200)
-    ref, cpu = run_ref_gpu(torch_cuda, case), run_cpu_oracle(case)
-    assert_matches_cpu_oracle(cpu, ref, case)
+    case = LARGE_CASES["scene60k_outside"]()
+    ref, cpu = refdata.reference("scene60k_outside", refdata.case_inputs(case)), run_cpu_oracle(case)
+    # common.assert_forward_close_cpu + the CPU gradient bar, on the stored entries of the reference's outputs
+    refdata.assert_equal(cpu["num_intersections"], ref["num_intersections"], "num_intersections")
+    refdata.assert_equal(cpu["depth_indices"], ref["depth_indices"], "depth_indices")
+    refdata.assert_close(cpu["rgba"], ref["rgba"], "rgba")
+    didx = ref["depth"].at(cpu["depth_indices"])  # equal to the reference's (checked above)
+    tol = common.depth_tolerance(case.foam.attributes, ref["depth"].values.astype(np.float64), didx)
+    bad = np.abs(ref["depth"].at(cpu["depth"]).astype(np.float64) - ref["depth"].values) > tol
+    assert not bad.any(), f"{int(bad.sum())} depth entries outside the conditioned bound"
+    refdata.assert_grads_close(cpu, ref, common.CPU_GRAD_TOL)
 
 
 def test_half_attributes_forward(torch_cuda):
     case = common.scene_case()
+    ref = refdata.reference("scene20k_half_forward", refdata.case_inputs(case))
     got = run_ours(torch_cuda, case, attr_dtype="float16", backward=False)
-    ref = run_ref_gpu(torch_cuda, case, attr_dtype="float16", backward=False)
     assert got["rgba"].dtype == np.float16
-    assert np.array_equal(got["num_intersections"], ref["num_intersections"])
-    assert np.array_equal(got["depth_indices"], ref["depth_indices"])
-    np.testing.assert_allclose(got["rgba"].astype(np.float32), ref["rgba"].astype(np.float32),
-                               rtol=1e-3, atol=1e-3)  # one half ulp
-    assert (got["rgba"] != ref["rgba"]).mean() < 1e-3
+    refdata.assert_equal(got["num_intersections"], ref["num_intersections"], "num_intersections")
+    refdata.assert_equal(got["depth_indices"], ref["depth_indices"], "depth_indices")
+    refdata.assert_close(got["rgba"], ref["rgba"], "rgba", rtol=1e-3, atol=1e-3)  # one half ulp
+    assert (ref["rgba"].at(got["rgba"]).astype(np.float64) != ref["rgba"].values).mean() < 1e-3
 
 
 def test_half_attributes_backward(torch_cuda):
@@ -259,55 +242,56 @@ def test_half_attributes_backward(torch_cuda):
     assert common.grad_error(got["attr_grad"].astype(np.float32), ref["attr_grad"].astype(np.float32)) < 2e-2
 
 
-@pytest.mark.parametrize("model", ["pinhole", "fisheye"])
-@pytest.mark.parametrize("attr_dtype", ["float16", "float32"])
-def test_trace_benchmark(torch_cuda, model, attr_dtype):
-    import radfoam_b200
-    from oracle import ref_gpu
+def benchmark_inputs(torch, model, attr_dtype):
+    """-> (scene tensors, camera dict, start cell) of test_trace_benchmark."""
     from radfoam_b200 import foam
 
-    if not ref_gpu.available():
-        pytest.skip("oracle/_ref not built")
-    torch = torch_cuda
     f = common.scene_case().foam
     attrs = f.attributes.astype(np.float16 if attr_dtype == "float16" else np.float32)
     scene = [to_dev(torch, x) for x in (f.points, attrs, f.adjacency, f.offsets)]
     pos = (2.5, 2.5, 2.5)
     cam = foam.camera_dict(pos, fov=0.9 if model == "pinhole" else 1.2, width=200, height=120, model=model)
     start = to_dev(torch, np.array([foam.nearest_point(f.points, pos)], dtype=np.uint32))
+    return scene, cam, start
+
+
+@pytest.mark.parametrize("model", ["pinhole", "fisheye"])
+@pytest.mark.parametrize("attr_dtype", ["float16", "float32"])
+def test_trace_benchmark(torch_cuda, model, attr_dtype):
+    import radfoam_b200
+
+    torch = torch_cuda
+    scene, cam, start = benchmark_inputs(torch, model, attr_dtype)
+    ref = refdata.reference(f"trace_benchmark_{model}_{attr_dtype}", (scene, cam, start))
     pipe = radfoam_b200.create_pipeline(3, attr_dtype)
     diff = pipe.prefetch_adjacent_diff(scene[0], scene[2], scene[3])
-    ref_diff = ref_gpu.prefetch_adjacent_diff(scene[0], scene[2], scene[3])
-    assert torch.equal(diff.view(torch.int16), ref_diff.view(torch.int16))
+    refdata.assert_equal(diff.view(torch.int16).cpu().numpy(), ref["adjacent_diff"], "prefetch_adjacent_diff")
     out = torch.zeros((120, 200), dtype=torch.uint32, device="cuda")
-    ref_out = torch.zeros((120, 200), dtype=torch.uint32, device="cuda")
     cam_t = {k: (torch.from_numpy(v) if isinstance(v, np.ndarray) else v) for k, v in cam.items()}
     pipe.trace_benchmark(*scene, diff, cam_t, start, out, weight_threshold=0.05)
-    ref_gpu.trace_benchmark(*scene, ref_diff, cam, start, ref_out, weight_threshold=0.05)
     torch.cuda.synchronize()
-    a = out.cpu().numpy().view(np.uint8).reshape(120, 200, 4).astype(np.int32)
-    b = ref_out.cpu().numpy().view(np.uint8).reshape(120, 200, 4).astype(np.int32)
-    assert np.array_equal(a, b), f"{int((a != b).any(axis=-1).sum())} pixels differ from the reference's bytes"
-    assert (b[..., :3].sum(axis=-1) > 0).mean() > 0.2  # the frame is not empty
+    frame = out.cpu().numpy()
+    refdata.assert_equal(frame, ref["frame"], "the frame's bytes")
+    a = frame.view(np.uint8).reshape(120, 200, 4).astype(np.int32)
+    assert (a[..., :3].sum(axis=-1) > 0).mean() > 0.2  # the frame is not empty
 
 
 # ------------------------------------------------------------------ walk tape (record / replay)
-@pytest.mark.parametrize("make_case", [lambda: common.config1(3, 2),
-                                       lambda: common.scene_case(num_points=60000, width=320, height=200),
-                                       lambda: common.scene_case(num_points=60000, width=320, height=200, inside=True),
-                                       lambda: common.random_ray_case(num_points=60000, num_rays=100000)],
+@pytest.mark.parametrize("make_case", [("config1_deg3_q2", lambda: common.config1(3, 2))]
+                         + list(LARGE_CASES.items()),
                          ids=["config1", "scene", "scene_inside", "random_batch"])
 def test_tape_replay_matches_reference_kernels(torch_cuda, make_case):
     """Forward that records the tape == plain forward bit for bit; backward that replays it ==
     the reference's re-walk backward."""
-    case = make_case()
+    name, make = make_case
+    case = make()
     got = run_ours(torch_cuda, case, tape=True)
     plain = run_ours(torch_cuda, case, tape=False)
     for k in ("rgba", "depth", "depth_indices", "num_intersections"):
         assert np.array_equal(got[k], plain[k]), k
-    ref = run_ref_gpu(torch_cuda, case)
-    assert_forward_equal(got, ref)
-    assert_grads_close(got, ref)
+    ref = refdata.reference(name, refdata.case_inputs(case))
+    refdata.assert_forward_equal(got, ref)
+    refdata.assert_grads_close(got, ref, GRAD_TOL)
 
 
 def test_tape_overflow_falls_back_then_grows(torch_cuda):
@@ -317,9 +301,8 @@ def test_tape_overflow_falls_back_then_grows(torch_cuda):
     import radfoam_b200
 
     torch = torch_cuda
-    case = common.scene_case(num_points=60000, width=320, height=200, inside=True)
-    ref = run_ref_gpu(torch, case)
-    assert ref["num_intersections"].max() > 40
+    case = LARGE_CASES["scene60k_inside"]()
+    ref = refdata.reference("scene60k_inside", refdata.case_inputs(case))
     f = case.foam
     pipe = radfoam_b200.create_pipeline(3)
     scene = [to_dev(torch, x) for x in (f.points, f.attributes, f.adjacency, f.offsets)]
@@ -332,8 +315,9 @@ def test_tape_overflow_falls_back_then_grows(torch_cuda):
         overflowed.append(pipe.tape_status()["overflowed"])
         bwd = pipe.trace_backward(*scene, rays, start, fwd["rgba"], g, dq, fwd["depth_indices"], gd)
         got = {k: v.cpu().numpy() for k, v in list(fwd.items()) + list(bwd.items()) if k != "ray_grad"}
-        assert_forward_equal(got, ref)
-        assert_grads_close(got, ref)
+        refdata.assert_forward_equal(got, ref)
+        refdata.assert_grads_close(got, ref, GRAD_TOL)
+        assert got["num_intersections"].max() > 40  # equal to the reference's: the scene needs two chunks
     assert overflowed[0] and not overflowed[-1], overflowed
     st = pipe.tape_status()
     assert st["used_chunks"] <= st["capacity_chunks"]
@@ -500,27 +484,22 @@ def test_validation_errors(torch_cuda):
 
 
 # ------------------------------------------------------------------ .pt checkpoint -> FPS loop (SURVEY.md §8f.3)
-def test_pt_checkpoint_benchmark_loop(torch_cuda, tmp_path):
-    """A scene saved in the reference's .pt layout, loaded as benchmark.py:36-38 does (fp16 attributes), rendered
-    through the FPS loop of benchmark.py:86-139; frames must equal direct trace_benchmark calls and, when
-    oracle/_ref is built, the reference kernel's frames (<= 1 level on a few pixels, as test_trace_benchmark)."""
+def pt_checkpoint_world(torch, directory):
+    """A scene saved in the reference's .pt layout and loaded as benchmark.py:36-38 does (fp16 attributes), the
+    cameras of benchmark.py's FPS loop, and what a direct trace_benchmark call of each camera needs."""
     import radfoam_b200
-    from oracle import ref_gpu
     from radfoam_b200 import foam, scene_io
 
-    torch = torch_cuda
     f = common.scene_case().foam
-    path = tmp_path / "model.pt"
+    path = os.path.join(directory, "model.pt")
     scene_io.FoamScene.from_foam(f, device="cpu").save_pt(path)
     scene = scene_io.FoamScene.load_pt(path, sh_degree=3, attr_dtype=torch.float16, device="cuda")
     width, height, fov = 160, 96, 0.9
     c2w = torch.zeros((17, 4, 4))
-    dicts = []
     for i in range(17):
         ang = 0.37 * i
         pos = (3.2 * np.cos(ang), 3.2 * np.sin(ang), 1.5)
         cam = foam.camera_dict(pos, fov=fov, width=width, height=height)
-        dicts.append(cam)
         c2w[i, :3, 0] = torch.from_numpy(cam["right"])
         c2w[i, :3, 1] = -torch.from_numpy(cam["up"])
         c2w[i, :3, 2] = torch.from_numpy(cam["forward"])
@@ -528,28 +507,38 @@ def test_pt_checkpoint_benchmark_loop(torch_cuda, tmp_path):
         c2w[i, 3, 3] = 1.0
     fy = height / (2.0 * np.tan(fov / 2.0))
     cameras, positions = scene_io.benchmark_cameras(c2w, fy, width, height)
-    assert len(cameras) == 3 and abs(cameras[0]["fov"] - fov) < 1e-6
     pipe = radfoam_b200.create_pipeline(3, "float16")
-    res = scene_io.benchmark_fps(pipe, scene, cameras, positions, n_reps=2)
+    trace_data = scene.get_trace_data()
+    points, _, adjacency, offsets = trace_data
+    return dict(scene=scene, width=width, height=height, fov=fov, cameras=cameras, positions=positions, pipe=pipe,
+                trace_data=trace_data, diff=pipe.prefetch_adjacent_diff(points, adjacency, offsets),
+                starts=radfoam_b200.nearest_point(points, positions.cuda()))
+
+
+def pt_checkpoint_inputs(w):
+    return w["trace_data"], w["cameras"], w["starts"], w["diff"]
+
+
+def test_pt_checkpoint_benchmark_loop(torch_cuda, tmp_path):
+    """A scene saved in the reference's .pt layout, loaded as benchmark.py:36-38 does (fp16 attributes), rendered
+    through the FPS loop of benchmark.py:86-139; frames must equal direct trace_benchmark calls and the reference
+    kernel's frames, byte for byte."""
+    from radfoam_b200 import scene_io
+
+    torch = torch_cuda
+    w = pt_checkpoint_world(torch, tmp_path)
+    height, width, cameras, pipe = w["height"], w["width"], w["cameras"], w["pipe"]
+    assert len(cameras) == 3 and abs(cameras[0]["fov"] - w["fov"]) < 1e-6
+    res = scene_io.benchmark_fps(pipe, w["scene"], cameras, w["positions"], n_reps=2)
     assert res["frames"] == 3 and res["fps"] > 0 and res["output"].shape == (3, height, width)
     frames = res["output"].cpu().numpy()
-    points, attributes, adjacency, offsets = scene.get_trace_data()
-    assert attributes.dtype == torch.float16
-    diff = pipe.prefetch_adjacent_diff(points, adjacency, offsets)
-    starts = radfoam_b200.nearest_point(points, positions.cuda())
-    for k, pose in enumerate((0, 8, 16)):
-        start = starts[k:k + 1]
+    assert w["trace_data"][1].dtype == torch.float16
+    ref = refdata.reference("pt_checkpoint_frames", pt_checkpoint_inputs(w))
+    for k in range(3):
         direct = torch.zeros((height, width), dtype=torch.uint32, device="cuda")
-        pipe.trace_benchmark(points, attributes, adjacency, offsets, diff, cameras[k], start, direct,
+        pipe.trace_benchmark(*w["trace_data"], w["diff"], cameras[k], w["starts"][k:k + 1], direct,
                              weight_threshold=0.05)
         assert np.array_equal(frames[k], direct.cpu().numpy())
         a = frames[k].view(np.uint8).reshape(height, width, 4).astype(np.int32)
         assert (a[..., :3].sum(axis=-1) > 0).mean() > 0.05         # the frame is not empty
-        if ref_gpu.available():
-            ref_out = torch.zeros((height, width), dtype=torch.uint32, device="cuda")
-            cam_np = {key: (v.numpy() if isinstance(v, torch.Tensor) else v) for key, v in cameras[k].items()}
-            ref_gpu.trace_benchmark(points, attributes, adjacency, offsets, diff, cam_np, start, ref_out,
-                                    weight_threshold=0.05)
-            torch.cuda.synchronize()
-            b = ref_out.cpu().numpy().view(np.uint8).reshape(height, width, 4).astype(np.int32)
-            assert np.array_equal(a, b), f"{int((a != b).any(axis=-1).sum())} pixels differ from the reference's bytes"
+        refdata.assert_equal(frames[k], ref[f"frame{k}"], f"frame {k}'s bytes")
